@@ -9,6 +9,7 @@ sync replicas, synthetic 28x28 data, random-init weights.  Weak scaling (per-GPU
     python bench.py --gpus N --steps K --warmup W          # our engine (N>1: under torchrun, or self-spawned)
     python bench.py --impl reference ...                   # the unmodified reference (unavailable here: TF1/py2)
     python bench.py --impl torch_ddp ...                   # baseline/: torch + cuDNN/cuBLAS + NCCL (for BASELINE.md)
+    python bench.py ... --dump-outputs DIR                 # also save the last timed step's results as DIR/*.npy
 
 One JSON line on stdout from rank 0.  Two measurements per run:
   * ``value``  -- K steps replayed from the CUDA graph with inputs already on the device, rotating through a
@@ -51,7 +52,31 @@ def parse_args():
     ap.add_argument("--kernel-times", action="store_true", help="also print per-kernel device times (stderr)")
     ap.add_argument("--trace", default="", help="after the timed runs: CUPTI timeline (torch.profiler) of a few graph-replayed "
                                                 "steps -> <path>.json (chrome trace) + <path>.txt (one step, kernel start/end)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps: rank 0's results of the last timed step -> DIR/loss_acc.npy (loss, "
+                         "accuracy) and DIR/params.npy (the updated fp32 weights; a fixed, seeded sample of %d of them "
+                         "when the model is larger), to compare two builds output for output; the weight gradients sum "
+                         "with fp32 atomics, so two runs agree closely, not bit for bit" % DUMP_MAX_PARAMS)
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_MAX_PARAMS = 8 << 20            # 32 MB of fp32 weights at most in a --dump-outputs directory
+
+
+def dump_outputs(out_dir: str, params, loss_acc) -> None:
+    """Write what a caller of the training step gets back: its (loss, accuracy) and the weights it left behind."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    flat = params.detach().float().cpu().reshape(-1)
+    if flat.numel() > DUMP_MAX_PARAMS:
+        idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_PARAMS].sort().values
+        flat = flat[idx]
+    np.save(os.path.join(out_dir, "params.npy"), flat.numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "loss_acc.npy"), np.asarray(loss_acc, dtype=np.float32).reshape(2))
 
 
 # ----------------------------------------------------------------------------------------------------
@@ -202,8 +227,9 @@ def main():
     d_pool = torch.empty(pool_n, h_pool[0].numel(), dtype=torch.uint8, device=ctx.device)
     for i in range(pool_n):
         d_pool[i].copy_(h_pool[i % n_host])
+    # drawn from the seeded generator too, not torch's process-wide one: identical inputs from run to run
     d_pool[:, :B * 784 * 4].view(torch.float32).view(pool_n, -1).add_(   # distinct images per pool entry
-        (torch.rand(pool_n, 1, device=ctx.device) - 0.5) * 0.1)
+        ((torch.rand(pool_n, 1, generator=g) - 0.5) * 0.1).to(ctx.device))
 
     def barrier():
         torch.cuda.synchronize()
@@ -310,6 +336,7 @@ def main():
     e0.record()
     pending = None
     last_loss = 0.0
+    last_loss_acc = None                                          # host buffer with the last timed step's (loss, accuracy)
     if k == n:
         for i in range(args.steps):
             ev = e2e_step(i)
@@ -319,13 +346,15 @@ def main():
             pending = ev
         pending[0].synchronize()
         last_loss = float(pending[1][0])
+        last_loss_acc = pending[1]
         images_e2e = n * B * args.steps
     else:
         def e2e_consume(i):
-            nonlocal last_loss
+            nonlocal last_loss, last_loss_acc
             ev = e2e_step(i)
             ev[0].synchronize()
             last_loss = float(ev[1][0])
+            last_loss_acc = ev[1]
         images_e2e = run_global_steps(e2e_consume, args.steps)
     e1.record()
     barrier()
@@ -334,6 +363,8 @@ def main():
         dist.all_reduce(ms2, op=dist.ReduceOp.MAX)
     ms2_total = float(ms2.item())
     backend.check_error()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, engine.params, last_loss_acc)
     info = engine.step_info()
     if args.kernel_times:
         kt = engine.time_kernels(20)

@@ -290,7 +290,9 @@ def check_bucketed_step_matches_single_kernel(B: int = 64, steps: int = 6, seed:
                 be = FusedBackend(ReplicaContext(0, 1, 0, torch.device("cuda", 0), "none"))
                 eng = CudaMlpEngine(model, B, be, hidden=hidden, seed=seed, use_graph=True)
             eng.use_graph = True
-            eng.attach_optimizer(SyncReplicasOptimizer(be, LearningRateSchedule(0.05, 2, 0.5), 1, 1))
+            # lr 0.01: on random labels at lr 0.05 a 1e-6 relative change of the gradients (fp32 atomics summing in another
+            # order) already moves the sixth loss by up to ~0.018, so the 0.02 loss bound below would sit inside that noise
+            eng.attach_optimizer(SyncReplicasOptimizer(be, LearningRateSchedule(0.01, 2, 0.5), 1, 1))
             losses = []
             p_init = eng.params.clone()
             for s in range(steps):
