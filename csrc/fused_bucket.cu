@@ -75,8 +75,9 @@ constexpr int EARLY2_THREADS = 128;
 // shard, SGD on the local fp32 master copy, bf16 shadow).  The LeNet step launches both at once; the MLP step launches the
 // exchange right after the big weight-gradient GEMM -- it touches neither weights nor shadow, so it may run next to the
 // data-gradient GEMM that still reads that layer's shadow -- and the apply after it.
-template <int NR>
-__global__ void __launch_bounds__(EARLY2_THREADS) bucket_early_kernel(SyncPeers P, SyncArgs a, BucketV2 r, int parts) {
+template <int NR, int RULE>
+__global__ void __launch_bounds__(EARLY2_THREADS) bucket_early_kernel(SyncPeers P, SyncArgs a, BucketV2 r, int parts, OptArgs o) {
+  using U = Update<RULE>;
   SyncCtrl* me = P.ctrl[a.rank];
   __shared__ uint32_t s_last;
   pdl_wait();
@@ -174,14 +175,16 @@ __global__ void __launch_bounds__(EARLY2_THREADS) bucket_early_kernel(SyncPeers 
     if (blockIdx.x == 0 && threadIdx.x == 0) me->t_phase_e[4] = globaltimer_ns();
   }
 
-  // ---- SGD on my fp32 master copy of fc1 from the (identical everywhere) bf16 gradient sum; fresh bf16 shadow ---------------
-  const float scale = device_lr(a, epoch) / (float)NR;
+  // ---- update my fp32 master copy of fc1 (and its local state) from the (identical everywhere) bf16 gradient sum; fresh bf16
+  // shadow ---------------------------------------------------------------------------------------------------------------
+  const U up(o, device_lr(a, epoch), (float)NR);
   float* w = P.params[a.rank] + 4 * (size_t)r.fc1_b4;
   __nv_bfloat16* sh = a.shadow != nullptr ? a.shadow + 4 * (size_t)r.fc1_b4 : nullptr;
-  constexpr int A = 2;
+  const size_t st4 = (size_t)r.fc1_b4;                                // fc1 inside the state arenas (float4 units)
+  constexpr int A = RULE == RULE_RMSPROP ? 1 : 2;                     // RMSProp's four state vectors: stay within 96 registers
   for (int c0 = tid; c0 < n8; c0 += A * stride) {
     uint4 g[A];
-    float4 w0[A], w1[A];
+    float4 w0[A], w1[A], sa0[A], sa1[A], sb0[A], sb1[A];
 #pragma unroll
     for (int u = 0; u < A; ++u) {
       const int c = c0 + u * stride;
@@ -189,17 +192,20 @@ __global__ void __launch_bounds__(EARLY2_THREADS) bucket_early_kernel(SyncPeers 
         g[u] = __ldcv(reinterpret_cast<const uint4*>(mine) + c);      // peers / the switch just wrote it: not through L1
         w0[u] = *reinterpret_cast<const float4*>(w + 8 * (size_t)c);
         w1[u] = *reinterpret_cast<const float4*>(w + 8 * (size_t)c + 4);
+        U::load(o, a.rank, st4 + 2 * (size_t)c, sa0[u], sb0[u]);
+        U::load(o, a.rank, st4 + 2 * (size_t)c + 1, sa1[u], sb1[u]);
       }
     }
 #pragma unroll
     for (int u = 0; u < A; ++u) {
       const int c = c0 + u * stride;
       if (c >= n8) continue;
-      float4 a0 = w0[u], a1 = w1[u];
-      a0.x -= scale * bf16_lo(g[u].x); a0.y -= scale * bf16_hi(g[u].x); a0.z -= scale * bf16_lo(g[u].y); a0.w -= scale * bf16_hi(g[u].y);
-      a1.x -= scale * bf16_lo(g[u].z); a1.y -= scale * bf16_hi(g[u].z); a1.z -= scale * bf16_lo(g[u].w); a1.w -= scale * bf16_hi(g[u].w);
+      const float4 a0 = up.step4(w0[u], make_float4(bf16_lo(g[u].x), bf16_hi(g[u].x), bf16_lo(g[u].y), bf16_hi(g[u].y)), sa0[u], sb0[u]);
+      const float4 a1 = up.step4(w1[u], make_float4(bf16_lo(g[u].z), bf16_hi(g[u].z), bf16_lo(g[u].w), bf16_hi(g[u].w)), sa1[u], sb1[u]);
       *reinterpret_cast<float4*>(w + 8 * (size_t)c) = a0;
       *reinterpret_cast<float4*>(w + 8 * (size_t)c + 4) = a1;
+      U::store(o, a.rank, st4 + 2 * (size_t)c, sa0[u], sb0[u]);
+      U::store(o, a.rank, st4 + 2 * (size_t)c + 1, sa1[u], sb1[u]);
       if (sh != nullptr)
         *reinterpret_cast<uint4*>(sh + 8 * (size_t)c) =
             make_uint4(pack_bf16x2(a0.x, a0.y), pack_bf16x2(a0.z, a0.w), pack_bf16x2(a1.x, a1.y), pack_bf16x2(a1.z, a1.w));
@@ -213,7 +219,9 @@ __global__ void __launch_bounds__(EARLY2_THREADS) bucket_early_kernel(SyncPeers 
 // ---------------------------------------------------------------------------------------------------------------------
 constexpr int LATE2_THREADS = 512;
 
-__global__ void __launch_bounds__(LATE2_THREADS, 1) bucket_late_kernel(SyncPeers P, SyncArgs a, BucketV2 r) {
+template <int RULE>
+__global__ void __launch_bounds__(LATE2_THREADS, 1) bucket_late_kernel(SyncPeers P, SyncArgs a, BucketV2 r, OptArgs o) {
+  using U = Update<RULE>;
   SyncCtrl* me = P.ctrl[a.rank];
   __shared__ uint32_t s_last;
   pdl_wait();
@@ -269,8 +277,8 @@ __global__ void __launch_bounds__(LATE2_THREADS, 1) bucket_late_kernel(SyncPeers
     publish_status(me, epoch + 1, me->accepted_steps + 1, me->dropped_steps, (NR >= 32) ? 0xffffffffu : ((1u << NR) - 1u), (uint32_t)NR, 0u);
   }
 
-  // ---- sum the N contributions in rank order, SGD on my copy, bf16 shadow --------------------------------------------------
-  const float scale = device_lr(a, epoch) / (float)NR;
+  // ---- sum the N contributions in rank order, update my copy (and my state), bf16 shadow ----------------------------------
+  const U up(o, device_lr(a, epoch), (float)NR);
   float* wdst = P.params[a.rank];
   const float* inbox = r.inbox[a.rank];
   for (int j = tid; j < n_late4; j += stride) {
@@ -282,13 +290,16 @@ __global__ void __launch_bounds__(LATE2_THREADS, 1) bucket_late_kernel(SyncPeers
       if (c < NR)
         g[c] = (c == a.rank) ? own : __ldcv(reinterpret_cast<const float4*>(inbox) + half + (size_t)c * (size_t)n_late4 + j);
     }
-    float4 nw = *reinterpret_cast<const float4*>(wdst + 4 * (size_t)i);
+    const float4 w0 = *reinterpret_cast<const float4*>(wdst + 4 * (size_t)i);
+    float4 sa, sb;
+    U::load(o, a.rank, (size_t)i, sa, sb);
     float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
     for (int c = 0; c < SYNC_MAX_RANKS; ++c)
       if (c < NR) { acc.x += g[c].x; acc.y += g[c].y; acc.z += g[c].z; acc.w += g[c].w; }
-    nw.x -= scale * acc.x; nw.y -= scale * acc.y; nw.z -= scale * acc.z; nw.w -= scale * acc.w;
+    const float4 nw = up.step4(w0, acc, sa, sb);
     *reinterpret_cast<float4*>(wdst + 4 * (size_t)i) = nw;
+    U::store(o, a.rank, (size_t)i, sa, sb);
     if (a.shadow != nullptr) {
       uint2 o;
       o.x = pack_bf16x2(nw.x, nw.y);
@@ -330,8 +341,9 @@ DMNIST_DEVICE uint4 ld_volatile_b128(const void* p) {
 // BF16 = true (default): a line carries FOUR gradients as bf16 -- {bf16x2, tag, bf16x2, tag} -- i.e. one line per float4, half the
 // bytes: at N = 8 every GPU ingests 7 slots, and 7 x 475 KB of fp32 lines were ~4 us of pure NVLink ingress on the critical path.
 // Every replica sums the SAME bf16-rounded contributions (its own included) in fp32, so the replicas stay bit-identical.
-template <bool BF16>
-__global__ void __launch_bounds__(LATE2_THREADS) bucket_late_ll_kernel(SyncPeers P, SyncArgs a, BucketV2 r) {
+template <bool BF16, int RULE>
+__global__ void __launch_bounds__(LATE2_THREADS) bucket_late_ll_kernel(SyncPeers P, SyncArgs a, BucketV2 r, OptArgs o) {
+  using U = Update<RULE>;
   SyncCtrl* me = P.ctrl[a.rank];
   pdl_wait();
   const uint32_t epoch = me->epoch;
@@ -380,8 +392,8 @@ __global__ void __launch_bounds__(LATE2_THREADS) bucket_late_ll_kernel(SyncPeers
     publish_status(me, epoch + 1, me->accepted_steps + 1, me->dropped_steps, (NR >= 32) ? 0xffffffffu : ((1u << NR) - 1u), (uint32_t)NR, 0u);
   }
 
-  // ---- receive: poll my inbox until the other replicas' lines of this step are there; rank-ordered sum; SGD; shadow -------
-  const float scale = device_lr(a, epoch) / (float)NR;
+  // ---- receive: poll my inbox until the other replicas' lines of this step are there; rank-ordered sum; update; shadow ----
+  const U up(o, device_lr(a, epoch), (float)NR);
   float* wdst = P.params[a.rank];
   const uint4* inbox = reinterpret_cast<const uint4*>(r.inbox[a.rank]);
   for (int j = tid; j < n_late4; j += stride) {
@@ -429,13 +441,16 @@ __global__ void __launch_bounds__(LATE2_THREADS) bucket_late_ll_kernel(SyncPeers
       for (int c = 0; c < SYNC_MAX_RANKS; ++c)
         if ((pending >> c) & 1u) g[c] = make_float4(0.f, 0.f, 0.f, 0.f);
     }
-    float4 nw = *reinterpret_cast<const float4*>(wdst + 4 * (size_t)i);
+    const float4 w0 = *reinterpret_cast<const float4*>(wdst + 4 * (size_t)i);
+    float4 sa, sb;
+    U::load(o, a.rank, (size_t)i, sa, sb);
     float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
     for (int c = 0; c < SYNC_MAX_RANKS; ++c)
       if (c < NR) { acc.x += g[c].x; acc.y += g[c].y; acc.z += g[c].z; acc.w += g[c].w; }
-    nw.x -= scale * acc.x; nw.y -= scale * acc.y; nw.z -= scale * acc.z; nw.w -= scale * acc.w;
+    const float4 nw = up.step4(w0, acc, sa, sb);
     *reinterpret_cast<float4*>(wdst + 4 * (size_t)i) = nw;
+    U::store(o, a.rank, (size_t)i, sa, sb);
     if (a.shadow != nullptr) {
       uint2 o;
       o.x = pack_bf16x2(nw.x, nw.y);
@@ -460,6 +475,47 @@ __global__ void __launch_bounds__(LATE2_THREADS) bucket_late_ll_kernel(SyncPeers
   }
 }
 
+template <int RULE>
+cudaError_t configure_bucket_kernels() {
+  cudaError_t e = cudaSuccess;
+  for (cudaError_t x : {set_max_shared_carveout(bucket_early_kernel<1, RULE>), set_max_shared_carveout(bucket_early_kernel<2, RULE>),
+                        set_max_shared_carveout(bucket_early_kernel<4, RULE>), set_max_shared_carveout(bucket_early_kernel<8, RULE>),
+                        set_max_shared_carveout(bucket_late_kernel<RULE>), set_max_shared_carveout(bucket_late_ll_kernel<true, RULE>),
+                        set_max_shared_carveout(bucket_late_ll_kernel<false, RULE>)})
+    if (e == cudaSuccess) e = x;
+  return e;
+}
+
+template <int RULE>
+int launch_bucket(const SyncPeers& P, const SyncArgs& a, const BucketV2& r, const OptArgs& o, int phase, int ctas,
+                  cudaStream_t stream, int late_ll, int late_bf16) {
+  const int nranks = a.nranks;
+  if (phase != 2) {
+    if (ctas < 1) ctas = 148;
+    const dim3 g(ctas), b(EARLY2_THREADS);
+    const int parts = phase == 1 ? 3 : (phase == 3 ? 1 : 2);
+    if (nranks == 1) return (int)launch_kernel(bucket_early_kernel<1, RULE>, g, b, 0, stream, P, a, r, parts, o);
+    if (nranks == 2) return (int)launch_kernel(bucket_early_kernel<2, RULE>, g, b, 0, stream, P, a, r, parts, o);
+    if (nranks == 4) return (int)launch_kernel(bucket_early_kernel<4, RULE>, g, b, 0, stream, P, a, r, parts, o);
+    if (nranks == 8) return (int)launch_kernel(bucket_early_kernel<8, RULE>, g, b, 0, stream, P, a, r, parts, o);
+    return -5;    // instantiated for 1, 2, 4 and 8 replicas; the caller falls back to the single kernel
+  }
+  if (nranks > 1 && r.inbox[0] == nullptr) return -3;
+  const int n_late4 = r.numel4 - (r.fc1_e4 - r.fc1_b4);
+  int grid = (n_late4 + LATE2_THREADS - 1) / LATE2_THREADS;      // one float4 per thread: a single round of loads
+  if (grid < 1) grid = 1;
+  // LL lines double the bytes and poll per element: the right protocol for a latency-bound SMALL bucket (LeNet: 236 KB); a
+  // large late bucket (the MLPs: megabytes) is bandwidth-bound and goes as plain data + release flags
+  if (late_ll && (long long)n_late4 * 16 <= (1ll << 20)) {        // no in-kernel barrier: any grid size is safe
+    if (grid > 296) grid = 296;
+    if (late_bf16) return (int)launch_kernel(bucket_late_ll_kernel<true, RULE>, dim3(grid), dim3(LATE2_THREADS), 0, stream, P, a, r, o);
+    return (int)launch_kernel(bucket_late_ll_kernel<false, RULE>, dim3(grid), dim3(LATE2_THREADS), 0, stream, P, a, r, o);
+  }
+  if (ctas >= 1 && grid > ctas) grid = ctas;
+  if (grid > 148) grid = 148;                                     // all CTAs must be co-resident (in-kernel barrier)
+  return (int)launch_kernel(bucket_late_kernel<RULE>, dim3(grid), dim3(LATE2_THREADS), 0, stream, P, a, r, o);
+}
+
 }  // namespace dm
 
 extern "C" {
@@ -474,9 +530,13 @@ extern "C" {
 int dm_bucket_sync(void* const* ctrl, void* const* params, void* const* grads, void* const* g16, void* const* inbox, int rank,
                    int nranks, int phase, long long fc1_begin, long long fc1_end, long long numel, float lr0,
                    float decay_rate, int decay_steps, double timeout_ms, void* shadow_bf16, int ctas, void* stream_,
-                   void* mc_g16, void* mc_inbox, int late_ll, int late_bf16) {
+                   void* mc_g16, void* mc_inbox, int late_ll, int late_bf16, int rule, void* const* s0, void* const* s1,
+                   float momentum, float decay, float eps) {
   using namespace dm;
   if (nranks < 1 || nranks > SYNC_MAX_RANKS || phase < 1 || phase > 4) return -1;
+  if (rule < RULE_SGD || rule > RULE_RMSPROP || (rule != RULE_SGD && s0 == nullptr) || (rule == RULE_RMSPROP && s1 == nullptr)) return -4;
+  // every rank updates its own state from the identical sums: no state crosses NVLink, no multicast views
+  const OptArgs o = make_opt_args(s0, s1, rank, nranks, nullptr, nullptr, momentum, decay, eps, 0.f);
   if ((fc1_begin & 7) || (fc1_end & 7) || (numel & 3) || fc1_begin < 0 || fc1_end < fc1_begin || fc1_end > numel) return -2;
   SyncPeers P;
   BucketV2 r;
@@ -501,39 +561,14 @@ int dm_bucket_sync(void* const* ctrl, void* const* params, void* const* grads, v
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
   static bool configured = false;
   if (!configured) {   // same L1/shared split as every other kernel of the step, or the CTAs cannot share an SM with them
-    DM_CUDA_OK(cudaFuncSetAttribute(bucket_early_kernel<1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    DM_CUDA_OK(cudaFuncSetAttribute(bucket_early_kernel<2>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    DM_CUDA_OK(cudaFuncSetAttribute(bucket_early_kernel<4>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    DM_CUDA_OK(cudaFuncSetAttribute(bucket_early_kernel<8>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    DM_CUDA_OK(cudaFuncSetAttribute(bucket_late_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    DM_CUDA_OK(cudaFuncSetAttribute(bucket_late_ll_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    DM_CUDA_OK(cudaFuncSetAttribute(bucket_late_ll_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    DM_CUDA_OK(configure_bucket_kernels<RULE_SGD>());
+    DM_CUDA_OK(configure_bucket_kernels<RULE_MOMENTUM>());
+    DM_CUDA_OK(configure_bucket_kernels<RULE_RMSPROP>());
     configured = true;
   }
-  if (phase != 2) {
-    if (ctas < 1) ctas = 148;
-    const dim3 g(ctas), b(EARLY2_THREADS);
-    const int parts = phase == 1 ? 3 : (phase == 3 ? 1 : 2);
-    if (nranks == 1) return (int)launch_kernel(bucket_early_kernel<1>, g, b, 0, stream, P, a, r, parts);
-    if (nranks == 2) return (int)launch_kernel(bucket_early_kernel<2>, g, b, 0, stream, P, a, r, parts);
-    if (nranks == 4) return (int)launch_kernel(bucket_early_kernel<4>, g, b, 0, stream, P, a, r, parts);
-    if (nranks == 8) return (int)launch_kernel(bucket_early_kernel<8>, g, b, 0, stream, P, a, r, parts);
-    return -5;    // instantiated for 1, 2, 4 and 8 replicas; the caller falls back to the single kernel
-  }
-  if (nranks > 1 && inbox == nullptr) return -3;
-  const int n_late4 = r.numel4 - (r.fc1_e4 - r.fc1_b4);
-  int grid = (n_late4 + LATE2_THREADS - 1) / LATE2_THREADS;      // one float4 per thread: a single round of loads
-  if (grid < 1) grid = 1;
-  // LL lines double the bytes and poll per element: the right protocol for a latency-bound SMALL bucket (LeNet: 236 KB); a
-  // large late bucket (the MLPs: megabytes) is bandwidth-bound and goes as plain data + release flags
-  if (late_ll && (long long)n_late4 * 16 <= (1ll << 20)) {        // no in-kernel barrier: any grid size is safe
-    if (grid > 296) grid = 296;
-    if (late_bf16) return (int)launch_kernel(bucket_late_ll_kernel<true>, dim3(grid), dim3(LATE2_THREADS), 0, stream, P, a, r);
-    return (int)launch_kernel(bucket_late_ll_kernel<false>, dim3(grid), dim3(LATE2_THREADS), 0, stream, P, a, r);
-  }
-  if (ctas >= 1 && grid > ctas) grid = ctas;
-  if (grid > 148) grid = 148;                                     // all CTAs must be co-resident (in-kernel barrier)
-  return (int)launch_kernel(bucket_late_kernel, dim3(grid), dim3(LATE2_THREADS), 0, stream, P, a, r);
+  if (rule == RULE_MOMENTUM) return launch_bucket<RULE_MOMENTUM>(P, a, r, o, phase, ctas, stream, late_ll, late_bf16);
+  if (rule == RULE_RMSPROP) return launch_bucket<RULE_RMSPROP>(P, a, r, o, phase, ctas, stream, late_ll, late_bf16);
+  return launch_bucket<RULE_SGD>(P, a, r, o, phase, ctas, stream, late_ll, late_bf16);
 }
 
 }  // extern "C"

@@ -15,8 +15,9 @@
 //                           replicas with count > 0 for this step, CAS the chief's commit word (exactly one winner, the
 //                           arrival-bitmap/commit ring of the K-of-N path), broadcast it, wait until no contributor is
 //                           mid-accumulate, re-read the counts: divisor = total number of accumulated gradients
-//   iv_apply     (grid)     winner only: sum the contributors' accumulators over NVLink (peer loads), x lr / total, SGD, push
-//                           the new weights into EVERY replica's arena (multimem.st / peer stores), release the "pushed" flags
+//   iv_apply     (grid)     winner only: sum the contributors' accumulators over NVLink (peer loads), / total, update rule,
+//                           push the new weights and optimizer state into EVERY replica's arenas (multimem.st / peer stores),
+//                           release the "pushed" flags
 //
 // A replica that is mid-iteration at the deadline is simply not in the mask (its count is 0) or contributes what it had; it
 // never waits for anybody and nobody waits for it.  Replicas hold bit-identical weights whenever no push is in flight.
@@ -163,14 +164,16 @@ __global__ void iv_close_kernel(SyncPeers P, SyncArgs a) {
   publish_status(me, me->epoch, me->accepted_steps, me->dropped_steps, me->last_mask, me->last_count, me->last_late);
 }
 
-__global__ void __launch_bounds__(IV_THREADS, 1) iv_apply_kernel(SyncPeers P, SyncArgs a, IntervalArgs r) {
+template <int RULE>
+__global__ void __launch_bounds__(IV_THREADS, 1) iv_apply_kernel(SyncPeers P, SyncArgs a, IntervalArgs r, OptArgs o) {
+  using U = Update<RULE>;
   SyncCtrl* me = P.ctrl[a.rank];
   __shared__ uint32_t s_last;
   pdl_wait();
   const uint32_t e = me->epoch;
   if (me->iv_commit_go != e + 1) return;
   const uint32_t mask = me->iv_commit_mask, total = me->iv_commit_total;
-  const float scale = device_lr(a, e) / (float)max(total, 1u);
+  const U up(o, device_lr(a, e), (float)max(total, 1u));
   int contrib[SYNC_MAX_RANKS];
   int nc = 0;
   for (int q = 0; q < a.nranks; ++q)
@@ -181,20 +184,25 @@ __global__ void __launch_bounds__(IV_THREADS, 1) iv_apply_kernel(SyncPeers P, Sy
 #pragma unroll
     for (int c = 0; c < SYNC_MAX_RANKS; ++c)
       g[c] = c < nc ? ld_peer_f4(r.acc[contrib[c]] + 4 * (size_t)i) : make_float4(0.f, 0.f, 0.f, 0.f);
-    float4 nw = *reinterpret_cast<const float4*>(wsrc + 4 * (size_t)i);
+    const float4 w0 = *reinterpret_cast<const float4*>(wsrc + 4 * (size_t)i);
+    float4 sa, sb;
+    U::load(o, a.rank, (size_t)i, sa, sb);
     float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
     for (int c = 0; c < SYNC_MAX_RANKS; ++c)
       if (c < nc) { s.x += g[c].x; s.y += g[c].y; s.z += g[c].z; s.w += g[c].w; }
-    nw.x -= scale * s.x; nw.y -= scale * s.y; nw.z -= scale * s.z; nw.w -= scale * s.w;
+    const float4 nw = up.step4(w0, s, sa, sb);
     if (a.mc_params != nullptr) {
       multimem_st_f4(a.mc_params + 4 * (size_t)i, nw);
       *reinterpret_cast<float4*>(P.params[a.rank] + 4 * (size_t)i) = nw;     // my own copy also through the local path
+      U::push(o, a.nranks, (size_t)i, sa, sb, true);
+      U::store(o, a.rank, (size_t)i, sa, sb);
     } else {
       for (int q = 0; q < a.nranks; ++q) st_peer_f4(P.params[q] + 4 * (size_t)i, nw);
+      U::push(o, a.nranks, (size_t)i, sa, sb, false);
     }
   }
-  // ---- all pushes are out -> publish the step ---------------------------------------------------------------------------------
+  // ---- all pushes (weights and state) are out -> publish the step ---------------------------------------------------------------------------------
   __syncthreads();
   if (threadIdx.x == 0) {
     fence_sc_sys();
@@ -236,9 +244,12 @@ int dm_interval_begin(void* ctrl, const void* params, void* shadow_bf16, long lo
 // Last four kernels of an interval-mode iteration: gate, accumulate, close (+ commit attempt), apply (winner only).
 int dm_interval_end(void* const* ctrl, void* const* params, void* const* grads, void* const* acc, int rank, int nranks,
                     long long numel, float lr0, float decay_rate, int decay_steps, double timeout_ms, int ctas, void* stream_,
-                    void* mc_params) {
+                    void* mc_params, int rule, void* const* s0, void* const* s1, void* mc_s0, void* mc_s1, float momentum,
+                    float decay, float eps) {
   using namespace dm;
   if (nranks < 1 || nranks > SYNC_MAX_RANKS || (numel & 3)) return -1;
+  if (rule < RULE_SGD || rule > RULE_RMSPROP || (rule != RULE_SGD && s0 == nullptr) || (rule == RULE_RMSPROP && s1 == nullptr)) return -4;
+  if (rule != RULE_SGD && nranks > 1 && mc_params != nullptr && (mc_s0 == nullptr || (rule == RULE_RMSPROP && mc_s1 == nullptr))) return -4;
   SyncPeers P;
   IntervalArgs r;
   for (int i = 0; i < SYNC_MAX_RANKS; ++i) {
@@ -255,6 +266,8 @@ int dm_interval_end(void* const* ctrl, void* const* params, void* const* grads, 
   a.timeout_ns = (unsigned long long)(timeout_ms * 1e6);
   a.shadow = nullptr; a.mc_grads = nullptr;
   a.mc_params = nranks > 1 ? reinterpret_cast<float*>(mc_params) : nullptr;
+  const OptArgs o = make_opt_args(s0, s1, rank, nranks, nranks > 1 ? mc_s0 : nullptr, nranks > 1 ? mc_s1 : nullptr,
+                                  momentum, decay, eps, 0.f);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream_);
   if (ctas < 1 || ctas > 148) ctas = 148;
   SyncCtrl* me = P.ctrl[rank];
@@ -265,7 +278,9 @@ int dm_interval_end(void* const* ctrl, void* const* params, void* const* grads, 
   if (e != cudaSuccess) return (int)e;
   e = launch_kernel(iv_close_kernel, dim3(1), dim3(32), 0, st, P, a);
   if (e != cudaSuccess) return (int)e;
-  return (int)launch_kernel(iv_apply_kernel, dim3(ctas), dim3(IV_THREADS), 0, st, P, a, r);
+  if (rule == RULE_MOMENTUM) return (int)launch_kernel(iv_apply_kernel<RULE_MOMENTUM>, dim3(ctas), dim3(IV_THREADS), 0, st, P, a, r, o);
+  if (rule == RULE_RMSPROP) return (int)launch_kernel(iv_apply_kernel<RULE_RMSPROP>, dim3(ctas), dim3(IV_THREADS), 0, st, P, a, r, o);
+  return (int)launch_kernel(iv_apply_kernel<RULE_SGD>, dim3(ctas), dim3(IV_THREADS), 0, st, P, a, r, o);
 }
 
 }  // extern "C"

@@ -107,8 +107,9 @@ DMNIST_DEVICE void decide(const SyncPeers& P, const SyncArgs& a, SyncCtrl* me, u
   }
 }
 
-template <bool KOFN>
-__global__ void __launch_bounds__(SYNC_THREADS, 1) fused_sync_sgd_kernel(SyncPeers P, SyncArgs a) {
+template <bool KOFN, int RULE>
+__global__ void __launch_bounds__(SYNC_THREADS, 1) fused_sync_sgd_kernel(SyncPeers P, SyncArgs a, OptArgs o) {
+  using U = Update<RULE>;
   SyncCtrl* me = P.ctrl[a.rank];
   __shared__ uint32_t s_mask, s_late, s_target, s_last;
   pdl_wait();      // the gradient arena is complete only when the backward kernels have finished
@@ -158,7 +159,7 @@ __global__ void __launch_bounds__(SYNC_THREADS, 1) fused_sync_sgd_kernel(SyncPee
     const int end = min(begin + shard, a.numel4);
     own_begin = begin;
     own_end = end;
-    const float scale = device_lr(a, epoch) / (float)count;
+    const U up(o, device_lr(a, epoch), (float)count);
     const uint32_t drop_thresh = a.drop_keep > 0.f ? (uint32_t)(a.drop_keep * 16777216.f) : 0u;
     int contrib[SYNC_MAX_RANKS];
     int nc = 0;
@@ -172,22 +173,23 @@ __global__ void __launch_bounds__(SYNC_THREADS, 1) fused_sync_sgd_kernel(SyncPee
       constexpr int V = 4;
       const int stride = gridDim.x * SYNC_THREADS;
       for (int i0 = begin + blockIdx.x * SYNC_THREADS + threadIdx.x; i0 < end; i0 += V * stride) {
-        float4 g[V], w[V];
+        float4 g[V], w[V], sa[V], sb[V];
 #pragma unroll
         for (int u = 0; u < V; ++u) {
           const int i = i0 + u * stride;
           if (i < end) {
             g[u] = multimem_ld_reduce_f4(a.mc_grads + 4 * (size_t)i);
             w[u] = *reinterpret_cast<const float4*>(wsrc + 4 * (size_t)i);
+            U::load(o, a.rank, (size_t)i, sa[u], sb[u]);
           }
         }
 #pragma unroll
         for (int u = 0; u < V; ++u) {
           const int i = i0 + u * stride;
           if (i >= end) continue;
-          float4 nw = w[u];
-          nw.x -= scale * g[u].x; nw.y -= scale * g[u].y; nw.z -= scale * g[u].z; nw.w -= scale * g[u].w;
+          const float4 nw = up.step4(w[u], g[u], sa[u], sb[u]);
           multimem_st_f4(a.mc_params + 4 * (size_t)i, nw);
+          U::push(o, a.nranks, (size_t)i, sa[u], sb[u], true);
           if (a.shadow != nullptr) {
             uint2 o;
             o.x = pack_bf16x2(nw.x, nw.y);
@@ -200,20 +202,23 @@ __global__ void __launch_bounds__(SYNC_THREADS, 1) fused_sync_sgd_kernel(SyncPee
     // Latency is the enemy here (a remote load is ~2 us): every thread issues the loads of ALL contributors
     // for U elements before it touches any of them, so one NVLink round trip covers the whole reduction of
     // its elements (at N = 8 a shard is so small that most threads make exactly one trip).
-    constexpr int U = 2;
+    constexpr int UN = 2;
     const int stride = gridDim.x * SYNC_THREADS;
-    for (int i0 = begin + blockIdx.x * SYNC_THREADS + threadIdx.x; i0 < end; i0 += U * stride) {
-      float4 g[U][SYNC_MAX_RANKS], w[U];
+    for (int i0 = begin + blockIdx.x * SYNC_THREADS + threadIdx.x; i0 < end; i0 += UN * stride) {
+      float4 g[UN][SYNC_MAX_RANKS], w[UN], sa[UN], sb[UN];
 #pragma unroll
-      for (int u = 0; u < U; ++u) {
+      for (int u = 0; u < UN; ++u) {
         const int i = i0 + u * stride;
 #pragma unroll
         for (int c = 0; c < SYNC_MAX_RANKS; ++c)
           g[u][c] = (c < nc && i < end) ? ld_peer_f4(P.grads[contrib[c]] + 4 * (size_t)i) : make_float4(0.f, 0.f, 0.f, 0.f);
-        if (i < end) w[u] = *reinterpret_cast<const float4*>(wsrc + 4 * (size_t)i);
+        if (i < end) {
+          w[u] = *reinterpret_cast<const float4*>(wsrc + 4 * (size_t)i);
+          U::load(o, a.rank, (size_t)i, sa[u], sb[u]);
+        }
       }
 #pragma unroll
-      for (int u = 0; u < U; ++u) {
+      for (int u = 0; u < UN; ++u) {
         const int i = i0 + u * stride;
         if (i >= end) continue;
         float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -231,9 +236,9 @@ __global__ void __launch_bounds__(SYNC_THREADS, 1) fused_sync_sgd_kernel(SyncPee
             acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
           }
         }
-        float4 nw = w[u];
-        nw.x -= scale * acc.x; nw.y -= scale * acc.y; nw.z -= scale * acc.z; nw.w -= scale * acc.w;
+        const float4 nw = up.step4(w[u], acc, sa[u], sb[u]);
         for (int q = 0; q < a.nranks; ++q) st_peer_f4(P.params[q] + 4 * (size_t)i, nw);
+        U::push(o, a.nranks, (size_t)i, sa[u], sb[u], false);
         if (a.shadow != nullptr) {   // my shard's bf16 shadow straight from registers
           uint2 o;
           o.x = pack_bf16x2(nw.x, nw.y);
@@ -580,9 +585,12 @@ int dm_sync_ctrl_offset(const char* field) {
 int dm_fused_sync_sgd(void* const* ctrl, void* const* params, void* const* grads, int rank, int nranks, int k,
                       long long numel, float lr0, float decay_rate, int decay_steps, float drop_keep,
                       unsigned int drop_seed, double timeout_ms, void* shadow_bf16, int ctas, void* stream_,
-                      const void* mc_grads, void* mc_params) {
+                      const void* mc_grads, void* mc_params, int rule, void* const* s0, void* const* s1, void* mc_s0,
+                      void* mc_s1, float momentum, float decay, float eps, float divisor) {
   using namespace dm;
   if (nranks < 1 || nranks > SYNC_MAX_RANKS || (numel & 3) || k < 1 || k > nranks) return -1;
+  if (rule < RULE_SGD || rule > RULE_RMSPROP || (rule != RULE_SGD && s0 == nullptr) || (rule == RULE_RMSPROP && s1 == nullptr)) return -4;
+  if (rule != RULE_SGD && mc_params != nullptr && (mc_s0 == nullptr || (rule == RULE_RMSPROP && mc_s1 == nullptr))) return -4;
   SyncPeers P;
   for (int i = 0; i < SYNC_MAX_RANKS; ++i) {
     const int j = i < nranks ? i : rank;
@@ -599,15 +607,27 @@ int dm_fused_sync_sgd(void* const* ctrl, void* const* params, void* const* grads
   a.mc_grads = reinterpret_cast<const float*>(mc_grads);
   a.mc_params = reinterpret_cast<float*>(mc_params);
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  const OptArgs o = make_opt_args(s0, s1, rank, nranks, mc_s0, mc_s1, momentum, decay, eps, divisor);
   if (ctas < 1) ctas = 64;
   static bool configured = false;
   if (!configured) {     // every kernel of the step runs with the same L1/shared split, so CTAs of different kernels can share an SM
-    DM_CUDA_OK(cudaFuncSetAttribute(fused_sync_sgd_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    DM_CUDA_OK(cudaFuncSetAttribute(fused_sync_sgd_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    DM_CUDA_OK(set_max_shared_carveout(fused_sync_sgd_kernel<true, RULE_SGD>));
+    DM_CUDA_OK(set_max_shared_carveout(fused_sync_sgd_kernel<false, RULE_SGD>));
+    DM_CUDA_OK(set_max_shared_carveout(fused_sync_sgd_kernel<true, RULE_MOMENTUM>));
+    DM_CUDA_OK(set_max_shared_carveout(fused_sync_sgd_kernel<false, RULE_MOMENTUM>));
+    DM_CUDA_OK(set_max_shared_carveout(fused_sync_sgd_kernel<true, RULE_RMSPROP>));
+    DM_CUDA_OK(set_max_shared_carveout(fused_sync_sgd_kernel<false, RULE_RMSPROP>));
     configured = true;
   }
-  if (k < nranks) return (int)launch_kernel(fused_sync_sgd_kernel<true>, dim3(ctas), dim3(SYNC_THREADS), 0, stream, P, a);
-  return (int)launch_kernel(fused_sync_sgd_kernel<false>, dim3(ctas), dim3(SYNC_THREADS), 0, stream, P, a);
+  const dim3 g(ctas), b(SYNC_THREADS);
+  switch (rule * 2 + (k < nranks ? 1 : 0)) {
+    case 2 * RULE_SGD + 1: return (int)launch_kernel(fused_sync_sgd_kernel<true, RULE_SGD>, g, b, 0, stream, P, a, o);
+    case 2 * RULE_MOMENTUM: return (int)launch_kernel(fused_sync_sgd_kernel<false, RULE_MOMENTUM>, g, b, 0, stream, P, a, o);
+    case 2 * RULE_MOMENTUM + 1: return (int)launch_kernel(fused_sync_sgd_kernel<true, RULE_MOMENTUM>, g, b, 0, stream, P, a, o);
+    case 2 * RULE_RMSPROP: return (int)launch_kernel(fused_sync_sgd_kernel<false, RULE_RMSPROP>, g, b, 0, stream, P, a, o);
+    case 2 * RULE_RMSPROP + 1: return (int)launch_kernel(fused_sync_sgd_kernel<true, RULE_RMSPROP>, g, b, 0, stream, P, a, o);
+    default: return (int)launch_kernel(fused_sync_sgd_kernel<false, RULE_SGD>, g, b, 0, stream, P, a, o);
+  }
 }
 
 // Bucketed aggregation, K == N.  phase 1 = early bucket [begin, end) floats, phase 2 = late bucket [begin, end) with the

@@ -177,6 +177,109 @@ DMNIST_DEVICE float device_lr(const SyncArgs& a, uint32_t step) {
   return a.lr0 * __powf(a.decay_rate, p);
 }
 
+// ---- update rules: the one place that spells the optimizer formulas for every aggregation kernel -----------------------
+// TF 1.x semantics (distributedmnist_b200/optim.py is the host twin):
+//   SGD       w -= lr * g
+//   MOMENTUM  a = momentum * a + g;  w -= lr * a                                       (ApplyMomentum, no Nesterov)
+//   RMSPROP   ms += (g * g - ms) * (1 - decay);  mom = momentum * mom + lr * g / sqrt(ms + eps);  w -= mom   (ApplyRMSProp)
+// with g = (sum over the contributors) / divisor.  The rule is a template parameter: the SGD instantiations compile to the
+// same instructions as the kernels had before state existed (the divisor stays folded into the rate there).
+enum : int { RULE_SGD = 0, RULE_MOMENTUM = 1, RULE_RMSPROP = 2 };
+
+// Per-parameter state: fp32 arenas with the parameter arena's layout, one per slot and rank (symmetric memory).
+struct OptArgs {
+  float* s0[SYNC_MAX_RANKS];    // momentum: accumulator a;  RMSProp: ms
+  float* s1[SYNC_MAX_RANKS];    // RMSProp: mom
+  float* mc_s0;                 // NVLS multicast views of the state arenas (set exactly when the parameter arena's is)
+  float* mc_s1;
+  float momentum, decay, eps;
+  float divisor;                // > 0: the mean's divisor instead of the contributor count (host-driven interval ticks)
+};
+
+template <int RULE>
+struct Update {
+  static constexpr int SLOTS = RULE == RULE_SGD ? 0 : (RULE == RULE_MOMENTUM ? 1 : 2);
+  float scale;                  // SGD: lr / count;  stateful rules: 1 / count (the mean is formed before the state sees it)
+  float lr, momentum, decay1, eps;
+
+  DMNIST_DEVICE Update(const OptArgs& o, float lr_, float count) {
+    if constexpr (RULE == RULE_SGD) {
+      scale = lr_ / count;
+      lr = momentum = decay1 = eps = 0.f;
+    } else {
+      scale = __frcp_rn(o.divisor > 0.f ? o.divisor : count);
+      lr = lr_;
+      momentum = o.momentum;
+      decay1 = 1.f - o.decay;
+      eps = o.eps;
+    }
+  }
+  // One element: `sum` = gradient sum over the contributors, `a` / `b` = its state slots.  Returns the new weight.
+  DMNIST_DEVICE float step(float w, float sum, float& a, float& b) const {
+    if constexpr (RULE == RULE_SGD) {
+      return w - scale * sum;
+    } else if constexpr (RULE == RULE_MOMENTUM) {
+      const float g = sum * scale;
+      a = momentum * a + g;
+      return w - lr * a;
+    } else {
+      const float g = sum * scale;
+      a += (g * g - a) * decay1;
+      b = momentum * b + __fdiv_rn(lr * g, __fsqrt_rn(a + eps));   // correctly rounded under --use_fast_math too
+      return w - b;
+    }
+  }
+  DMNIST_DEVICE float4 step4(float4 w, float4 s, float4& a, float4& b) const {
+    w.x = step(w.x, s.x, a.x, b.x);
+    w.y = step(w.y, s.y, a.y, b.y);
+    w.z = step(w.z, s.z, a.z, b.z);
+    w.w = step(w.w, s.w, a.w, b.w);
+    return w;
+  }
+  // state of arena float4 `i` in replica `r`'s arenas
+  DMNIST_DEVICE static void load(const OptArgs& o, int r, size_t i, float4& a, float4& b) {
+    if constexpr (SLOTS > 0) a = reinterpret_cast<const float4*>(o.s0[r])[i];
+    if constexpr (SLOTS > 1) b = reinterpret_cast<const float4*>(o.s1[r])[i];
+  }
+  DMNIST_DEVICE static void store(const OptArgs& o, int r, size_t i, float4 a, float4 b) {
+    if constexpr (SLOTS > 0) reinterpret_cast<float4*>(o.s0[r])[i] = a;
+    if constexpr (SLOTS > 1) reinterpret_cast<float4*>(o.s1[r])[i] = b;
+  }
+  // the owner of a shard replicates its new state into every replica's arenas, next to the weights: multicast (NVLS) or
+  // peer stores.  Must be issued before the fence that precedes the owner's "pushed" flag.
+  DMNIST_DEVICE static void push(const OptArgs& o, int nranks, size_t i, float4 a, float4 b, bool multicast) {
+    if constexpr (SLOTS > 0) {
+      if (multicast) multimem_st_f4(o.mc_s0 + 4 * i, a);
+      else for (int q = 0; q < nranks; ++q) st_peer_f4(o.s0[q] + 4 * i, a);
+    }
+    if constexpr (SLOTS > 1) {
+      if (multicast) multimem_st_f4(o.mc_s1 + 4 * i, b);
+      else for (int q = 0; q < nranks; ++q) st_peer_f4(o.s1[q] + 4 * i, b);
+    }
+  }
+};
+
+// Every kernel of the step runs with the same L1/shared split, so CTAs of different kernels can share an SM.
+template <class Kern>
+inline cudaError_t set_max_shared_carveout(Kern kern) {
+  return cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+}
+
+// Pointer tables of the state arenas (index = rank, like SyncPeers), hyper-parameters, divisor override.
+inline OptArgs make_opt_args(void* const* s0, void* const* s1, int rank, int nranks, void* mc_s0, void* mc_s1,
+                             float momentum, float decay, float eps, float divisor) {
+  OptArgs o;
+  for (int i = 0; i < SYNC_MAX_RANKS; ++i) {
+    const int j = i < nranks ? i : rank;
+    o.s0[i] = s0 != nullptr ? reinterpret_cast<float*>(s0[j]) : nullptr;
+    o.s1[i] = s1 != nullptr ? reinterpret_cast<float*>(s1[j]) : nullptr;
+  }
+  o.mc_s0 = reinterpret_cast<float*>(mc_s0);
+  o.mc_s1 = reinterpret_cast<float*>(mc_s1);
+  o.momentum = momentum; o.decay = decay; o.eps = eps; o.divisor = divisor;
+  return o;
+}
+
 // Poll (RELAXED loads inside pred) until pred() or the watchdog fires, then ONE acquire load of the flag the wait was about
 // (`acq`: LDG.STRONG.SYS + a single CCTL.IVALL; a fence.acq_rel.sys here would be a MEMBAR.ALL.SYS, which also waits for every
 // outstanding store of the SM -- measured: +4 us per step at N = 2 -- and an acquire load on every poll invalidates the SM's

@@ -36,6 +36,7 @@ from .models import get_model
 from .models.lenet import dropout_seed_mix
 from .ops import gemm as G
 from .ops.lib import check, load, ptr, stream_ptr
+from .optim import rule_or_sgd
 from .parallel.backends import StepInfo
 from .parallel.fused import FusedBackend
 
@@ -233,8 +234,13 @@ class CudaLeNetEngine(ComputeEngine):
         """Bind the aggregation policy so the whole step (compute + fused sync) is one graph."""
         sched = opt.lr_schedule
         k = getattr(opt, "replicas_to_aggregate", opt.total_num_replicas)
+        # update rule + its state arenas (symmetric, parameter-arena layout, NVLS-mapped when the fabric has multicast): the
+        # optimizer owns them, every aggregation launch of the step reads and writes them
+        rule = rule_or_sgd(getattr(opt, "update_rule", None))
+        slots = opt.ensure_slots(self.spec.arena_numel) if rule.num_slots else []
+        self.slots = slots
         self._opt_args = dict(k=int(k), lr0=float(sched.initial_learning_rate), decay_rate=float(sched.decay_rate),
-                              decay_steps=int(sched.decay_steps))
+                              decay_steps=int(sched.decay_steps), rule=rule, slots=slots)
         if getattr(opt, "drop_connect_probability", None) is not None:
             self.backend.drop_connect_(self.grads, opt.drop_connect_probability, 0)
         self._straggler = getattr(opt, "_straggler", None)
@@ -257,7 +263,8 @@ class CudaLeNetEngine(ComputeEngine):
         can = (hasattr(self, "_bucket_split") and int(k) == n and self._branches and self.backend.drop_keep <= 0.0
                and getattr(opt, "mode", "") != "interval")
         self._bucket_v2 = can and mode == "2" and n in (1, 2, 4, 8)
-        self._bucketed = can and ((mode == "1" and n in (2, 4, 8)) or self._bucket_v2)
+        # the round-1 bucket kernels apply SGD only: a stateful rule takes the single kernel there
+        self._bucketed = can and ((mode == "1" and n in (2, 4, 8) and rule.num_slots == 0) or self._bucket_v2)
         if self._bucket_v2 and self._g16 is None:
             e0, e1 = self._bucket_early
             assert e0 % 8 == 0 and (e1 - e0) % 8 == 0, "fc1 weights must start on a 32-byte boundary of the arena"
@@ -365,7 +372,7 @@ class CudaLeNetEngine(ComputeEngine):
                 if self._bucket_v2:
                     self.backend.enqueue_bucket_v2(self.params, self.grads, self._g16, self._inbox, 1, e0, e1, oa["lr0"],
                                                    oa["decay_rate"], oa["decay_steps"], ctas=self._early_ctas,
-                                                   stream=self._side[0])
+                                                   stream=self._side[0], rule=oa["rule"], slots=oa["slots"])
                 else:
                     self.backend.enqueue_bucket(self.params, self.grads, 1, e0, e1, e0, e1, oa["lr0"], oa["decay_rate"],
                                                 oa["decay_steps"], ctas=self._early_ctas, stream=self._side[0])
@@ -514,7 +521,7 @@ class CudaLeNetEngine(ComputeEngine):
             e0, e1 = self._bucket_early
             if self._bucket_v2:
                 self.backend.enqueue_bucket_v2(self.params, self.grads, self._g16, self._inbox, 2, e0, e1, oa["lr0"],
-                                               oa["decay_rate"], oa["decay_steps"])
+                                               oa["decay_rate"], oa["decay_steps"], rule=oa["rule"], slots=oa["slots"])
             else:
                 self.backend.enqueue_bucket(self.params, self.grads, 2, 0, self.spec.arena_numel, e0, e1,
                                             oa["lr0"], oa["decay_rate"], oa["decay_steps"])
@@ -525,7 +532,8 @@ class CudaLeNetEngine(ComputeEngine):
                 n += 1
             if interval:
                 oa = self._opt_args
-                self.backend.enqueue_interval_end(self.params, self.grads, self._acc, oa["lr0"], oa["decay_rate"], oa["decay_steps"])
+                self.backend.enqueue_interval_end(self.params, self.grads, self._acc, oa["lr0"], oa["decay_rate"], oa["decay_steps"],
+                                                  rule=oa["rule"], slots=oa["slots"])
                 n += 4
             else:
                 self.backend.enqueue(self.params, self.grads, **self._opt_args)
@@ -743,7 +751,7 @@ class CudaMlpEngine(ComputeEngine):
                 side = self._side[0]
                 side.wait_event(ev)
                 be.enqueue_bucket_v2(self.params, self.grads, self._g16, self._inbox, 3 if i > 1 else 1, e0, e1, oa["lr0"],
-                                     oa["decay_rate"], oa["decay_steps"], stream=side)
+                                     oa["decay_rate"], oa["decay_steps"], stream=side, rule=oa["rule"], slots=oa["slots"])
                 n += 1
                 if i == 1:
                     self._join_early = torch.cuda.Event()
@@ -763,7 +771,7 @@ class CudaMlpEngine(ComputeEngine):
                     side = self._side[0]
                     side.wait_event(ev2)
                     be.enqueue_bucket_v2(self.params, self.grads, self._g16, self._inbox, 4, e0, e1, oa["lr0"],
-                                         oa["decay_rate"], oa["decay_steps"], stream=side)
+                                         oa["decay_rate"], oa["decay_steps"], stream=side, rule=oa["rule"], slots=oa["slots"])
                     n += 1
                     self._join_early = torch.cuda.Event()
                     self._join_early.record(side)
@@ -799,7 +807,7 @@ class CudaMlpEngine(ComputeEngine):
             oa = self._opt_args
             e0, e1 = self._bucket_early
             self.backend.enqueue_bucket_v2(self.params, self.grads, self._g16, self._inbox, 2, e0, e1, oa["lr0"],
-                                           oa["decay_rate"], oa["decay_steps"])
+                                           oa["decay_rate"], oa["decay_steps"], rule=oa["rule"], slots=oa["slots"])
             n += 1
         elif with_sync:
             if self._straggler is not None:
@@ -807,7 +815,8 @@ class CudaMlpEngine(ComputeEngine):
                 n += 1
             if interval:
                 oa = self._opt_args
-                self.backend.enqueue_interval_end(self.params, self.grads, self._acc, oa["lr0"], oa["decay_rate"], oa["decay_steps"])
+                self.backend.enqueue_interval_end(self.params, self.grads, self._acc, oa["lr0"], oa["decay_rate"], oa["decay_steps"],
+                                                  rule=oa["rule"], slots=oa["slots"])
                 n += 4
             else:
                 self.backend.enqueue(self.params, self.grads, **self._opt_args)

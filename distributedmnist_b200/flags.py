@@ -63,6 +63,7 @@ class FlagValues:
     def __init__(self) -> None:
         object.__setattr__(self, "_flags", {})
         object.__setattr__(self, "_parsed", False)
+        object.__setattr__(self, "_validators", [])
 
     # ---- definition -----------------------------------------------------
     def _define(self, kind: str, name: str, default: Any, help: str) -> None:
@@ -89,6 +90,10 @@ class FlagValues:
 
     def DEFINE_string(self, name: str, default: str, help: str = "") -> None:
         self._define("string", name, default, help)
+
+    def register_validator(self, check: Callable[["FlagValues"], None]) -> None:
+        """``check(flags)`` runs after every :meth:`parse`; a ``ValueError`` it raises becomes a :class:`FlagError`."""
+        self._validators.append(check)
 
     # ---- access ---------------------------------------------------------
     def __getattr__(self, name: str) -> Any:
@@ -177,6 +182,11 @@ class FlagValues:
                 text = text[1:-1]
             f.value = f.parse(text)
             f.present = True
+        for check in self._validators:
+            try:
+                check(self)
+            except ValueError as e:
+                raise FlagError(str(e)) from None
         object.__setattr__(self, "_parsed", True)
         return rest
 
@@ -253,7 +263,20 @@ def define_engine_flags(F: FlagValues = FLAGS) -> FlagValues:
                                              "(page-locked result buffers, background batch packer)")
     F.DEFINE_integer("log_every", 1, "Log every n-th local iteration (1 = reference behaviour)")
     F.DEFINE_float("dropout_keep_prob", 0.5, "Keep probability of the fc1 dropout (reference mnist.py:139)")
+    # update rule of every aggregation path (distributedmnist_b200/optim.py); the defaults are the reference's otherwise
+    # unused RMSProp constants (src/distributed_train.py:102-104)
+    F.DEFINE_string("optimizer", "sgd", "sgd | momentum | rmsprop (TF 1.x ApplyGradientDescent / ApplyMomentum / ApplyRMSProp)")
+    F.DEFINE_float("momentum", 0.9, "Momentum of --optimizer=momentum and of RMSProp's momentum term, in [0, 1)")
+    F.DEFINE_float("rmsprop_decay", 0.9, "RMSProp decay of the mean square, in [0, 1)")
+    F.DEFINE_float("rmsprop_epsilon", 1.0, "RMSProp epsilon, > 0")
+    if _check_optimizer_flags not in F._validators:
+        F.register_validator(_check_optimizer_flags)
     return F
+
+
+def _check_optimizer_flags(F: FlagValues) -> None:
+    from .optim import check_hyper
+    check_hyper(F.optimizer, float(F.momentum), float(F.rmsprop_decay), float(F.rmsprop_epsilon))
 
 
 define_reference_flags()

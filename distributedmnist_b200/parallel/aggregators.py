@@ -27,6 +27,7 @@ from typing import Callable, Dict, List, Optional
 
 import torch
 
+from ..optim import UpdateRule, rule_or_sgd
 from .backends import Backend, StepInfo
 
 
@@ -49,8 +50,11 @@ def parse_straggler_spec(text: str) -> Dict[int, StragglerSpec]:
 
 class _AggregatorBase:
     def __init__(self, backend: Backend, lr_schedule: Callable[[int], float], total_num_replicas: int,
-                 straggler: Optional[Dict[int, StragglerSpec]] = None, seed: int = 0):
+                 straggler: Optional[Dict[int, StragglerSpec]] = None, seed: int = 0,
+                 update_rule: Optional[UpdateRule] = None):
         self.backend = backend
+        self.update_rule = rule_or_sgd(update_rule)
+        self.slots: List[torch.Tensor] = []     # optimizer state arenas (parameter-arena layout), see ensure_slots()
         self.lr_schedule = lr_schedule
         self.total_num_replicas = int(total_num_replicas)
         self.local_step = 0          # global step of the weights my next gradient is computed from (X7)
@@ -64,11 +68,23 @@ class _AggregatorBase:
     def global_step(self) -> int:
         return self.local_step
 
+    def ensure_slots(self, numel: int) -> List[torch.Tensor]:
+        """The update rule's state arenas, allocated through the backend (symmetric memory on the fused backend) and set to
+        their initial values on first use.  Every rank calls it in the same order (the allocation may be collective)."""
+        if len(self.slots) != self.update_rule.num_slots:
+            self.slots = self.update_rule.allocate_slots(self.backend.allocate, numel)
+        return self.slots
+
     def _delay_s(self) -> float:
         s = self._straggler
         if s is not None and self._rng.random() < s.prob:
             return s.usec * 1e-6
         return 0.0
+
+    def _rule_kw(self, params: torch.Tensor) -> dict:
+        if self.update_rule.num_slots == 0:
+            return {}          # SGD: the backends' call is exactly what it was before state existed
+        return dict(rule=self.update_rule, slots=self.ensure_slots(params.numel()))
 
     def _account(self, info: StepInfo) -> StepInfo:
         self.last_info = info
@@ -93,8 +109,9 @@ class SyncReplicasOptimizer(_AggregatorBase):
     """Mode A: synchronous SGD that commits on the first K of N gradients."""
 
     def __init__(self, backend: Backend, lr_schedule, replicas_to_aggregate: int, total_num_replicas: int,
-                 drop_connect_probability: Optional[float] = None, straggler=None, seed: int = 0):
-        super().__init__(backend, lr_schedule, total_num_replicas, straggler, seed)
+                 drop_connect_probability: Optional[float] = None, straggler=None, seed: int = 0,
+                 update_rule: Optional[UpdateRule] = None):
+        super().__init__(backend, lr_schedule, total_num_replicas, straggler, seed, update_rule)
         if not 1 <= replicas_to_aggregate <= total_num_replicas:
             raise ValueError("replicas_to_aggregate=%d must be in [1, %d]" % (replicas_to_aggregate, total_num_replicas))
         self.replicas_to_aggregate = int(replicas_to_aggregate)
@@ -118,7 +135,7 @@ class SyncReplicasOptimizer(_AggregatorBase):
         grads = self._drop_connect(grads)
         lr = self.lr_schedule(self.local_step)
         info = self.backend.sync_step(params, grads, lr, self.local_step, self.replicas_to_aggregate,
-                                      delay_s=self._delay_s())
+                                      delay_s=self._delay_s(), **self._rule_kw(params))
         return self._account(info)
 
 
@@ -127,8 +144,8 @@ class TimeoutReplicasOptimizer(_AggregatorBase):
 
     def __init__(self, backend: Backend, lr_schedule, total_num_replicas: int, mode: str = "cdf",
                  interval_ms: int = 1000, straggler=None, seed: int = 0,
-                 clock: Callable[[], float] = time.monotonic):
-        super().__init__(backend, lr_schedule, total_num_replicas, straggler, seed)
+                 clock: Callable[[], float] = time.monotonic, update_rule: Optional[UpdateRule] = None):
+        super().__init__(backend, lr_schedule, total_num_replicas, straggler, seed, update_rule)
         assert mode in ("cdf", "interval")
         self.mode = mode
         self.interval_s = interval_ms / 1000.0
@@ -175,7 +192,7 @@ class TimeoutReplicasOptimizer(_AggregatorBase):
         if self.mode == "cdf":
             lr = self.lr_schedule(self.local_step)
             info = self.backend.sync_step(params, grads, lr, self.local_step, self.total_num_replicas,
-                                          delay_s=self._delay_s())
+                                          delay_s=self._delay_s(), **self._rule_kw(params))
             return self._account(info)
         # interval: push into the local accumulator, never block on other replicas
         # until a deadline has passed.
@@ -193,7 +210,7 @@ class TimeoutReplicasOptimizer(_AggregatorBase):
             # tick) -- missed deadlines are skipped, never replayed, and no replica decides on its own to run another tick
             # (reference: the chief's timer sleeps the interval after each take_grad, …modified.py:208-215).
             lr = self.lr_schedule(self.local_step)
-            res = self.backend.interval_tick(params, self._acc, self._acc_count, lr, self._tick)
+            res = self.backend.interval_tick(params, self._acc, self._acc_count, lr, self._tick, **self._rule_kw(params))
             chief_now = getattr(self.backend, "last_chief_clock", None)
             nxt = self._tick + 1
             if chief_now is not None and self._t0 is not None:

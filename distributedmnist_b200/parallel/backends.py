@@ -16,8 +16,10 @@ The *policy* (K-of-N / full barrier / interval, SURVEY §2.3) lives in
   elementwise kernel).
 
 All backends honour the same contract: after ``sync_step`` every replica holds
-bit-identical parameters, the divisor is the number of accepted gradients, and
-late/stale gradients are discarded without stalling the update.
+bit-identical parameters (and optimizer state), the divisor is the number of
+accepted gradients, and late/stale gradients are discarded without stalling the
+update.  ``rule`` (``optim.UpdateRule``, None = SGD) and ``slots`` (its state
+arenas, laid out like ``params``) select and carry the update rule.
 """
 from __future__ import annotations
 
@@ -28,6 +30,7 @@ from typing import List, Optional
 import torch
 import torch.distributed as dist
 
+from ..optim import rule_or_sgd
 from .context import ReplicaContext
 from .protocol import Decision, StoreCommitBoard
 
@@ -71,11 +74,11 @@ class Backend:
 
     # -- hot path -----------------------------------------------------------
     def sync_step(self, params: torch.Tensor, grads: torch.Tensor, lr: float, local_step: int,
-                  k: int, delay_s: float = 0.0) -> StepInfo:
+                  k: int, delay_s: float = 0.0, rule=None, slots=()) -> StepInfo:
         raise NotImplementedError
 
     def interval_tick(self, params: torch.Tensor, acc: torch.Tensor, count: int, lr: float,
-                      tick: int) -> StepInfo:
+                      tick: int, rule=None, slots=()) -> StepInfo:
         raise NotImplementedError
 
 
@@ -86,17 +89,17 @@ class LocalBackend(Backend):
         super().__init__(ctx)
         self._global_step = 0
 
-    def sync_step(self, params, grads, lr, local_step, k, delay_s=0.0) -> StepInfo:
+    def sync_step(self, params, grads, lr, local_step, k, delay_s=0.0, rule=None, slots=()) -> StepInfo:
         if delay_s > 0:
             time.sleep(delay_s)
-        params.add_(grads, alpha=-float(lr))
+        rule_or_sgd(rule).apply(params, grads, 1, lr, slots)
         self._global_step = local_step + 1
         return StepInfo(self._global_step, True, 1, 1)
 
-    def interval_tick(self, params, acc, count, lr, tick) -> StepInfo:
+    def interval_tick(self, params, acc, count, lr, tick, rule=None, slots=()) -> StepInfo:
         if count == 0:
             return StepInfo(self._global_step, False, 0, 0, applied=False)
-        params.add_(acc, alpha=-float(lr) / count)
+        rule_or_sgd(rule).apply(params, acc, count, lr, slots)
         self._global_step += 1
         return StepInfo(self._global_step, True, 1, count)
 
@@ -129,18 +132,18 @@ class _CollectiveBackend(Backend):
             self._board.gc(local_step - 8)
         return d
 
-    def sync_step(self, params, grads, lr, local_step, k, delay_s=0.0) -> StepInfo:
+    def sync_step(self, params, grads, lr, local_step, k, delay_s=0.0, rule=None, slots=()) -> StepInfo:
         d = self._decide(local_step, k, delay_s)
         # Masked contribution: a late replica joins the collective with zeros, so
         # the sum holds exactly the accepted gradients and everyone divides by the
         # same popcount -- replicas stay bit-identical.
         contrib = grads if d.accepted else torch.zeros_like(grads)
         dist.all_reduce(contrib, op=dist.ReduceOp.SUM)
-        params.add_(contrib, alpha=-float(lr) / d.count)
+        rule_or_sgd(rule).apply(params, contrib, d.count, lr, slots)
         self._global_step = d.global_step
         return StepInfo(d.global_step, d.accepted, d.mask, d.count, stale=d.stale)
 
-    def interval_tick(self, params, acc, count, lr, tick) -> StepInfo:
+    def interval_tick(self, params, acc, count, lr, tick, rule=None, slots=()) -> StepInfo:
         cnt = torch.tensor([float(count)], dtype=torch.float32, device=acc.device)
         dist.all_reduce(cnt, op=dist.ReduceOp.SUM)
         total = int(cnt.item())
@@ -150,7 +153,7 @@ class _CollectiveBackend(Backend):
         if total == 0:
             return StepInfo(self._global_step, False, 0, 0, applied=False)
         dist.all_reduce(acc, op=dist.ReduceOp.SUM)
-        params.add_(acc, alpha=-float(lr) / total)
+        rule_or_sgd(rule).apply(params, acc, total, lr, slots)
         self._global_step += 1
         return StepInfo(self._global_step, count > 0, mask, total)
 

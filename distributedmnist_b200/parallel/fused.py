@@ -3,9 +3,10 @@
 The product path for SURVEY §2.5 X1-X8: the parameter arena, the gradient arena and a
 control block live in symmetric memory; one kernel per step publishes arrival, obtains
 the commit mask (all-to-all flags for K == N, chief-owned bitmap + CAS for K < N), sums
-the contributors' gradients straight out of peer HBM over NVLink, scales by
-``lr / popcount(mask)``, applies SGD on its shard and pushes the new weights into every
-rank's arena, then refreshes the local bf16 shadow used by the tensor-core kernels.
+the contributors' gradients straight out of peer HBM over NVLink, divides by
+``popcount(mask)``, applies the update rule (SGD, momentum or RMSProp, ``optim.py``) on
+its shard and pushes the new weights -- and the rule's state -- into every rank's arenas,
+then refreshes the local bf16 shadow used by the tensor-core kernels.
 No NCCL collective and no separate elementwise kernel is launched.
 
 Two ways to drive it:
@@ -24,6 +25,7 @@ from typing import Dict, List, Optional
 import torch
 
 from ..ops.lib import check, load, require_blackwell, stream_ptr
+from ..optim import rule_or_sgd
 from .backends import Backend, StepInfo
 from .context import ReplicaContext
 from .symm_mem import SymmetricBuffer, allocate_symmetric
@@ -211,19 +213,35 @@ class FusedBackend(Backend):
         return [(int(ts[s % ring]), int(ta[s % ring])) for s in range(first_step, last_step + 1)]
 
     # ---- launches -------------------------------------------------------------------------------
+    def _state_args(self, rule, slots, multicast: bool):
+        """C arguments of the update rule: code, the two state-arena pointer tables, their multicast views (only when the
+        weights travel by multicast too), momentum, decay, epsilon."""
+        rule = rule_or_sgd(rule)
+        if len(slots) != rule.num_slots:
+            raise ValueError("update rule %s keeps %d state arenas, got %d" % (rule.name, rule.num_slots, len(slots)))
+        bufs = [self._by_ptr[t.data_ptr()] for t in slots] + [None, None]
+        tables = [b.ptr_table() if b is not None else None for b in bufs[:2]]
+        mc = [ctypes.c_void_p(b.multicast_ptr if (multicast and b is not None) else 0) for b in bufs[:2]]
+        return [int(rule.code)] + tables + mc + [ctypes.c_float(x) for x in rule.hyper]
+
     def enqueue(self, params: torch.Tensor, grads: torch.Tensor, k: int, lr0: float, decay_rate: float = 1.0,
-                decay_steps: int = 1, stream: Optional[torch.cuda.Stream] = None) -> None:
+                decay_steps: int = 1, stream: Optional[torch.cuda.Stream] = None, rule=None, slots=(),
+                divisor: float = 0.0) -> None:
+        """``rule`` / ``slots``: update rule and its state arenas (symmetric, from :meth:`allocate`); ``divisor`` > 0 replaces
+        the contributor count as the mean's divisor (stateful rules only)."""
         pb, gb = self._by_ptr[params.data_ptr()], self._by_ptr[grads.data_ptr()]
+        mcg, mcp = self._mc_ptrs(pb, gb, slots)
         rc = self.lib.dm_fused_sync_sgd(
             self.ctrl.ptr_table(), pb.ptr_table(), gb.ptr_table(), self.ctx.rank, self.ctx.world_size, int(k),
             ctypes.c_longlong(params.numel()), ctypes.c_float(lr0), ctypes.c_float(decay_rate), int(decay_steps),
             ctypes.c_float(self.drop_keep), ctypes.c_uint(self.drop_seed), ctypes.c_double(self.timeout_ms),
             ctypes.c_void_p(0 if self.shadow is None else self.shadow.data_ptr()), int(self.ctas), stream_ptr(stream),
-            *self._mc_ptrs(pb, gb))
+            mcg, mcp, *self._state_args(rule, slots, bool(mcp.value)), ctypes.c_float(divisor))
         check(rc, "dm_fused_sync_sgd")
 
-    def _mc_ptrs(self, pb, gb):
-        on = self.use_nvls and pb.multicast_ptr and gb.multicast_ptr
+    def _mc_ptrs(self, pb, gb, slots=()):
+        on = self.use_nvls and pb.multicast_ptr and gb.multicast_ptr \
+            and all(self._by_ptr[t.data_ptr()].multicast_ptr for t in slots)
         return ctypes.c_void_p(gb.multicast_ptr if on else 0), ctypes.c_void_p(pb.multicast_ptr if on else 0)
 
     def enqueue_bucket(self, params: torch.Tensor, grads: torch.Tensor, phase: int, begin: int, end: int,
@@ -242,10 +260,11 @@ class FusedBackend(Backend):
 
     def enqueue_bucket_v2(self, params: torch.Tensor, grads: torch.Tensor, g16, inbox, phase: int, fc1_begin: int,
                           fc1_end: int, lr0: float, decay_rate: float = 1.0, decay_steps: int = 1, ctas: int = 0,
-                          stream: Optional[torch.cuda.Stream] = None) -> None:
+                          stream: Optional[torch.cuda.Stream] = None, rule=None, slots=()) -> None:
         """Bucketed aggregation, bf16 wire (csrc/fused_bucket.cu).  ``phase`` 1: reduce the bf16 fc1 gradient buffer ``g16``
-        in place over NVLink (NVLS or P2P) and apply SGD to the local fp32 fc1 weights -- a side branch of the step graph;
-        ``phase`` 2: push the small bucket into every replica's ``inbox``, sum in rank order, SGD, close the step."""
+        in place over NVLink (NVLS or P2P) and apply the update rule to the local fp32 fc1 weights and state -- a side
+        branch of the step graph; ``phase`` 2: push the small bucket into every replica's ``inbox``, sum in rank order,
+        update, close the step.  Every rank updates its own state from the identical sums: state never crosses NVLink."""
         pb, gb = self._by_ptr[params.data_ptr()], self._by_ptr[grads.data_ptr()]
         on = self.use_nvls and self.ctx.world_size > 1
         mc_g16 = g16.multicast_ptr if on else 0
@@ -256,7 +275,8 @@ class FusedBackend(Backend):
             ctypes.c_longlong(fc1_begin), ctypes.c_longlong(fc1_end), ctypes.c_longlong(params.numel()),
             ctypes.c_float(lr0), ctypes.c_float(decay_rate), int(decay_steps), ctypes.c_double(self.timeout_ms),
             ctypes.c_void_p(0 if self.shadow is None else self.shadow.data_ptr()), int(ctas), stream_ptr(stream),
-            ctypes.c_void_p(mc_g16), ctypes.c_void_p(mc_inbox), int(self.late_ll), int(self.late_bf16))
+            ctypes.c_void_p(mc_g16), ctypes.c_void_p(mc_inbox), int(self.late_ll), int(self.late_bf16),
+            *[x for i, x in enumerate(self._state_args(rule, slots, False)) if i not in (3, 4)])
         check(rc, "dm_bucket_sync(phase %d)" % phase)
 
     # ---- device-side interval mode (mode C, csrc/fused_interval.cu) ----------------------------------------------------------
@@ -276,15 +296,18 @@ class FusedBackend(Backend):
 
     def enqueue_interval_end(self, params: torch.Tensor, grads: torch.Tensor, acc: torch.Tensor, lr0: float,
                              decay_rate: float = 1.0, decay_steps: int = 1,
-                             stream: Optional[torch.cuda.Stream] = None) -> None:
+                             stream: Optional[torch.cuda.Stream] = None, rule=None, slots=()) -> None:
         """End of an interval-mode iteration: accumulate the gradient locally; after the tick's deadline try to commit the
-        tick (mean of whatever every replica has accumulated) -- never blocks on another replica's progress."""
+        tick (mean of whatever every replica has accumulated) -- never blocks on another replica's progress.  The committer
+        pushes the new weights and the rule's state into every replica."""
         pb, gb, ab = self._by_ptr[params.data_ptr()], self._by_ptr[grads.data_ptr()], self._by_ptr[acc.data_ptr()]
-        mc = pb.multicast_ptr if (self.use_nvls and pb.multicast_ptr) else 0
+        on = self.use_nvls and pb.multicast_ptr and all(self._by_ptr[t.data_ptr()].multicast_ptr for t in slots)
+        mc = pb.multicast_ptr if on else 0
         check(self.lib.dm_interval_end(self.ctrl.ptr_table(), pb.ptr_table(), gb.ptr_table(), ab.ptr_table(), self.ctx.rank,
                                        self.ctx.world_size, ctypes.c_longlong(params.numel()), ctypes.c_float(lr0),
                                        ctypes.c_float(decay_rate), int(decay_steps), ctypes.c_double(self.timeout_ms),
-                                       int(self.ctas), stream_ptr(stream), ctypes.c_void_p(mc)), "dm_interval_end")
+                                       int(self.ctas), stream_ptr(stream), ctypes.c_void_p(mc),
+                                       *self._state_args(rule, slots, bool(mc))), "dm_interval_end")
 
     @property
     def nvls_active(self) -> bool:
@@ -323,13 +346,13 @@ class FusedBackend(Backend):
         return StepInfo(global_step=st["epoch"], accepted=not late, mask=st["last_mask"], count=st["last_count"],
                         stale=bool(late))
 
-    def sync_step(self, params, grads, lr, local_step, k, delay_s: float = 0.0) -> StepInfo:
+    def sync_step(self, params, grads, lr, local_step, k, delay_s: float = 0.0, rule=None, slots=()) -> StepInfo:
         if delay_s > 0:
             self.enqueue_straggler_delay(1.0, delay_s * 1e6)
-        self.enqueue(params, grads, k, lr0=float(lr))
+        self.enqueue(params, grads, k, lr0=float(lr), rule=rule, slots=slots)
         return self.last_step_info(check=True)   # one device -> host read (synchronises)
 
-    def interval_tick(self, params, acc, count, lr, tick) -> StepInfo:
+    def interval_tick(self, params, acc, count, lr, tick, rule=None, slots=()) -> StepInfo:
         """Mode C tick: every rank joins; ranks with an empty accumulator contribute zeros and the
         divisor is the total number of accumulated gradients (mean of whatever arrived)."""
         counts = self.all_gather_object(int(count))
@@ -337,8 +360,12 @@ class FusedBackend(Backend):
         mask = sum(1 << i for i, c in enumerate(counts) if c > 0)
         if total == 0:
             return StepInfo(self.device_epoch, False, 0, 0, applied=False)
-        # lr/total instead of lr/popcount: fold the ratio into lr0 (kernel divides by N contributors)
-        self.enqueue(params, acc, self.ctx.world_size, lr0=float(lr) * self.ctx.world_size / total)
+        if rule_or_sgd(rule).num_slots == 0:
+            # lr/total instead of lr/popcount: fold the ratio into lr0 (kernel divides by N contributors)
+            self.enqueue(params, acc, self.ctx.world_size, lr0=float(lr) * self.ctx.world_size / total)
+        else:
+            # with state the mean has to be formed before the rule sees it: pass the divisor itself
+            self.enqueue(params, acc, self.ctx.world_size, lr0=float(lr), rule=rule, slots=slots, divisor=float(total))
         info = self.last_step_info()
         self.check_error()
         return StepInfo(info.global_step, count > 0, mask, total)

@@ -30,6 +30,7 @@ import torch
 from .checkpoint import Saver
 from .engine import make_engine
 from .flags import FLAGS
+from .optim import UpdateRule
 from .parallel.aggregators import (SyncReplicasOptimizer, TimeoutReplicasOptimizer,
                                    parse_straggler_spec)
 from .parallel.backends import make_backend
@@ -47,11 +48,13 @@ LOG_FORMAT = ("Worker %d: %s: step %d, loss = %f, train_acc = %f, test_acc = %f"
 
 
 class _AsyncCheckpointer:
-    """Chief-side saver: snapshot on the training thread, file IO on a helper thread."""
+    """Chief-side saver: snapshot on the training thread, file IO on a helper thread.  The optimizer's state arenas are
+    snapshotted at the same drained point as the weights and saved under TF's slot names (``Variable_4/Momentum``)."""
 
-    def __init__(self, train_dir: str, spec, interval_s: float, step_fn=None):
+    def __init__(self, train_dir: str, spec, interval_s: float, step_fn=None, opt=None):
         self.train_dir, self.spec, self.interval_s = train_dir, spec, interval_s
         self.step_fn = step_fn       # GPU path: drain the step in flight and read the device step counter (consistent snapshot)
+        self.opt = opt               # update rule + state arenas (opt.slots)
         self.saver = Saver()
         self._next = time.time() + interval_s
         self._thread: Optional[threading.Thread] = None
@@ -65,6 +68,8 @@ class _AsyncCheckpointer:
         if self.step_fn is not None:
             global_step = self.step_fn()         # the host loop runs one step ahead of what it has consumed
         state = self.spec.to_state_dict(params)  # consistent snapshot (device -> host copy)
+        if self.opt is not None and self.opt.update_rule.num_slots:
+            state.update(self.opt.update_rule.slots_to_state_dict(self.spec, self.opt.ensure_slots(params.numel())))
         if self._thread is not None:
             self._thread.join()
         self._thread = threading.Thread(target=self.saver.save, args=(self.train_dir, state, global_step))
@@ -159,23 +164,26 @@ def train(ctx: ReplicaContext, dataset, dataset_test=None, flags=FLAGS) -> Dict:
     spec = engine.spec
     lr_schedule = LearningRateSchedule.from_flags(flags, dataset.num_examples, num_replicas_to_aggregate)
     straggler = parse_straggler_spec(flags.inject_straggler)
+    rule = UpdateRule.from_flags(flags)
 
     if flags.interval_method or flags.worker_times_cdf_method:
         # reference :179-183 -- interval wins when both are set, as there.
         mode = "interval" if flags.interval_method else "cdf"
         opt = TimeoutReplicasOptimizer(backend, lr_schedule, total_num_replicas=num_workers, mode=mode,
-                                       interval_ms=flags.interval_ms, straggler=straggler, seed=flags.seed)
+                                       interval_ms=flags.interval_ms, straggler=straggler, seed=flags.seed,
+                                       update_rule=rule)
     else:
         opt = SyncReplicasOptimizer(
             backend, lr_schedule, replicas_to_aggregate=num_replicas_to_aggregate,
             total_num_replicas=num_workers,
             drop_connect_probability=flags.drop_connect_probability if flags.drop_connect else None,
-            straggler=straggler, seed=flags.seed)
+            straggler=straggler, seed=flags.seed, update_rule=rule)
     # GPU path: every mode runs as one CUDA graph per step -- K-of-N / full barrier through the fused aggregation kernels,
     # interval through the device-side deadline protocol (csrc/fused_interval.cu)
     fused_step = hasattr(engine, "attach_optimizer")
     if fused_step:
         engine.attach_optimizer(opt)   # GPU path: compute + fused allreduce/SGD replay as one CUDA graph
+    slots = opt.ensure_slots(spec.arena_numel) if rule.num_slots else []   # optimizer state, initial values
 
     # Supervisor semantics: chief restores the newest checkpoint, everyone gets it.
     restored_step = 0
@@ -186,10 +194,20 @@ def train(ctx: ReplicaContext, dataset, dataset_test=None, flags=FLAGS) -> Dict:
             state, restored_step = Saver.restore(latest)
             engine.params.copy_(spec.from_state_dict(state).to(engine.params.device))
             log.info("Restored model from %s at step=%d" % (latest, restored_step))
+            if slots:
+                if rule.has_slots(spec, state):
+                    for t, flat in zip(slots, rule.slots_from_state_dict(spec, state)):
+                        t.copy_(flat.to(t.device))
+                    log.info("Restored %s optimizer slots (%s)" % (rule.name, ", ".join(rule.slot_names)))
+                else:
+                    log.info("Checkpoint has no %s optimizer slots (%s): they start from their initial values"
+                             % (rule.name, ", ".join(rule.slot_names)))
     if num_workers > 1:
         restored_step = backend.all_gather_object(restored_step)[0]
         if restored_step > 0:
             backend.broadcast_(engine.params, 0)
+            for t in slots:
+                backend.broadcast_(t, 0)
     if restored_step > 0:
         opt.local_step = restored_step
         if hasattr(backend, "set_global_step"):
@@ -202,7 +220,7 @@ def train(ctx: ReplicaContext, dataset, dataset_test=None, flags=FLAGS) -> Dict:
         torch.cuda.synchronize()
         return int(backend.device_epoch)
     ckpt = _AsyncCheckpointer(flags.train_dir, spec, flags.save_interval_secs,
-                              step_fn=_device_step if (fused_step and hasattr(backend, "device_epoch")) else None) \
+                              step_fn=_device_step if (fused_step and hasattr(backend, "device_epoch")) else None, opt=opt) \
         if is_chief else None
     summary = SummaryWriter(flags.train_dir) if (is_chief and flags.should_summarize) else None
 
